@@ -375,6 +375,32 @@ def gemm_roofline(dev, M, N=256, K=256, what="GCN layer product of a padded batc
             "note": "arithmetic intensity 2*256/(2+2+~0) ~ 128 FLOP/B < ridge ~250: the HBM roofline applies"}
 
 
+# ------------------------------------------------------------------------------------------------ outputs
+DUMP_SAMPLE = 1 << 23           # parameter entries written by --dump-outputs (32 MB in float32)
+
+
+def dump_outputs(out_dir, model, loss_sum, n_tokens):
+    """What the timed step hands its caller, read after the last timed step: the loss sum and token count it returns
+    (loss_sum.npy, n_tokens.npy, float64) and the parameters Adam left (parameters.npy, float32).  Written by rank 0.
+    Through the CUDA-graph engine (the default) the loss sum and token count are rank 0's own, over its shard of the
+    global batch; through the eager --no-graph step they are global: the step's mean loss times its global token
+    count, and that count.  Compare dumps taken with the same flags and world size.  The parameters are
+    concatenated in model.parameters() order and sampled at DUMP_SAMPLE sorted positions drawn by numpy's generator
+    with seed 0 (torch's generator is left alone: it seeds the dropout of the legs that follow).  Atomic gradient
+    reductions make two runs of one build differ in the last bits, and Adam's normalised update magnifies that on
+    entries whose gradient is near zero: compare dumps with a tolerance."""
+    import numpy as np
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    flat = torch.cat([p.detach().reshape(-1) for p in model.parameters()])
+    n = flat.numel()
+    idx = torch.from_numpy(np.sort(np.random.default_rng(0).choice(n, min(n, DUMP_SAMPLE), replace=False)))
+    arrays = {"loss_sum": loss_sum.double(), "n_tokens": n_tokens.double(),
+              "parameters": flat[idx.to(flat.device)].float()}
+    for name, t in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), t.cpu().numpy())
+
+
 # ------------------------------------------------------------------------------------------------ GPU arm
 def run_gpu_arm(args):
     import torch
@@ -454,6 +480,7 @@ def run_gpu_arm(args):
         return ms.item()
 
     last_loss = [0.0]
+    last_step = [None]                  # what the last timed step returned, for --dump-outputs
     if args.graph:
         # whole step captured in a CUDA graph (fira_icse_b200/engine.py): one cudaGraphLaunch per step
         eng = GraphedTrainStep(model, B, adam_factory(model),
@@ -469,7 +496,7 @@ def run_gpu_arm(args):
         optimizer, bucket = eng.optimizer, eng.bucket
 
         def resident_step(i):
-            eng.step(pool_dev[i % N_POOL])
+            last_step[0] = eng.step(pool_dev[i % N_POOL])            # (loss sum, token count)
 
         def e2e_step(i):
             eng.step(host_list(pool_host[i % N_POOL]))               # pinned host -> static device buffers -> replay
@@ -482,7 +509,7 @@ def run_gpu_arm(args):
         launches_per_step = None
 
         def resident_step(i):
-            dp.step(pool_dev[i % N_POOL])
+            last_step[0] = dp.step(pool_dev[i % N_POOL])             # (mean loss, token count)
 
         def e2e_step(i):
             loss, _ = dp.step(device_batch(pool_host[i % N_POOL], dev, B))
@@ -499,6 +526,9 @@ def run_gpu_arm(args):
     launches = (_lib.LAUNCH_COUNT - launches0) if launches_per_step is None else launches_per_step * args.steps
     clocks = sampler.stop() if rank == 0 else None
     value = world * B * args.steps / (ms * 1e-3)
+    if args.dump_outputs and rank == 0:
+        loss, n_tok = last_step[0]
+        dump_outputs(args.dump_outputs, model, loss if args.graph else loss * n_tok, n_tok)
 
     if args.timeline:
         from torch.profiler import ProfilerActivity, profile
@@ -710,7 +740,14 @@ def main():
     ap.add_argument("--profile-step", action="store_true",
                     help="profiling runs only (ncu --profile-from-start off): after the timed region, ONE more step "
                          "between cudaProfilerStart/Stop, then exit without the extra legs")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one computed to DIR/<name>.npy (see dump_outputs) "
+                         "so that two builds can be compared output for output")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to the CUDA path (--impl ours)")
+    if args.dump_outputs and args.steps < 1:
+        ap.error("--dump-outputs writes what the last timed step computed: it needs --steps 1 or more")
     if not args.graph and args.layout == "packed":
         args.layout = "trimmed"                      # eager launches (profiling runs): the padded layout
     if args.impl == "reference":
